@@ -2,6 +2,7 @@
 """Benchmark of the EGNN forward hot path (BASELINE.json metric: node-pairs/sec, dim=512 N=1024).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|eager] [--dtype bf16|fp32]
+                    [--dump-outputs DIR]
 
 One "step" = one EGNN(dim=512) layer forward over one batch (B=4 graphs x N=1024 nodes, dense
 all-pairs = 4,194,304 node pairs) of synthetic N(0,1) inputs with the reference's default init
@@ -23,6 +24,11 @@ reference in PyTorch eager on the same B200 (the ">= 10x" comparison of BASELINE
 `--impl reference` times the reference's own torch CPU forward (kind "reference"; if baseline/_ref is
 absent, oracle/egnn_torch_port.py -- a torch restatement with the same ATen call sequence -- and kind
 "port"), all host threads, one graph of the same B=4 x N=1024 workload per step.
+
+`--dump-outputs DIR` (with `--impl ours`) writes the (feats, coors) the module returned in the last timed step as
+DIR/feats.npy and DIR/coors.npy, in float32 (exact for bf16 and fp32 outputs; 8 MiB for c2).  Module and inputs
+come from fixed seeds, so two builds run with the same arguments can be compared output for output.  Under
+torchrun each rank runs its own batch; rank r > 0 writes feats_rank<r>.npy and coors_rank<r>.npy.
 """
 from __future__ import annotations
 
@@ -36,6 +42,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the source tree, which may be read-only
 REPO = os.path.dirname(os.path.abspath(__file__))
 for p in (REPO, os.path.join(REPO, "tests")):
     if p not in sys.path:
@@ -439,10 +446,15 @@ def arm_ours(args):
     for a, b in evs:
         flush.zero_()                      # L2 flush between timed iterations (not timed)
         a.record()
-        mod(f_dev, x_dev)
+        last = mod(f_dev, x_dev)
         b.record()
     sync_all()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:
+        suffix = f"_rank{rank}" if rank else ""
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in zip(("feats", "coors"), last):
+            np.save(os.path.join(args.dump_outputs, f"{name}{suffix}.npy"), t.float().cpu().numpy())
     ms_total = sum(a.elapsed_time(b) for a, b in evs)
     ms = (C.c_float * 4)(); spans = (C.c_int32 * 4)(); launches = C.c_int64()
     lib.egnn_profile_read(ms, spans, C.byref(launches), 1)
@@ -602,7 +614,13 @@ def main():
     ap.add_argument("--dtype", default="bf16", choices=["bf16", "fp32"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--lean", action="store_true", help="metric, e2e and roofline only (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the (feats, coors) of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "cpu-sample":
         print(json.dumps(cpu_sample(args.workload)))
         return
