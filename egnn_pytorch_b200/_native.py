@@ -178,9 +178,9 @@ def strerror(code: int) -> str:
 
 
 class EgnnNativeError(RuntimeError):
-    def __init__(self, fn, code):
+    def __init__(self, fn, code, detail=None):
         self.code = code
-        super().__init__(f"{fn} failed: {strerror(code)} (code {code})")
+        super().__init__(f"{fn} failed: {strerror(code)} (code {code})" + (f": {detail}" if detail else ""))
 
 
 def check(fn: str, code: int):

@@ -31,10 +31,25 @@ inline BwdWs bwd_ws_layout(const Dims& s, const SimtPackLayout& L, size_t es, ui
   return w;
 }
 
+// Dynamic shared memory of the larger of bwd1 and the bwd2 variant launch_pair_bwd picks (the same size functions
+// the launches use).  The dense recompute (launch_tiled_recompute) is left out: it falls back by itself.
+template <typename T>
+inline size_t backward_smem_bytes(const Dims& s, uint32_t flags) {
+  const SimtPackLayout L = simt_pack_layout(s);
+  const bool knn = s.k > 0;
+  const int R = rec_layout(s, L.MP).R;
+  const size_t b1 = bwd1_smem_bytes<T>(s, L, knn, (flags & EGNN_FLAG_SOFT_EDGES) != 0);
+  const size_t b2 = knn ? bwd2_knn_smem_bytes<T>(s, R) : bwd2_dense_smem_bytes<T>(s, R);
+  return std::max(b1, b2);
+}
+
 inline int backward_supported(const EgnnLayerDesc& d) {
   if (d.dtype != EGNN_DTYPE_F32 && d.dtype != EGNN_DTYPE_F64) return EGNN_ERR_UNSUPPORTED;
   if (!(d.row_begin == 0 && (d.row_end == 0 || d.row_end == d.N))) return EGNN_ERR_UNSUPPORTED;
   if (d.label_dim > 0 && d.num_labels > BW2_MAXLAB) return EGNN_ERR_UNSUPPORTED;
+  const Dims s = make_dims(d);
+  const size_t smem = d.dtype == EGNN_DTYPE_F64 ? backward_smem_bytes<double>(s, d.flags) : backward_smem_bytes<float>(s, d.flags);
+  if (smem > DYN_SMEM_MAX) return EGNN_ERR_UNSUPPORTED;     // ensure_dynamic_smem would refuse it at launch
   return EGNN_OK;
 }
 

@@ -60,11 +60,15 @@ static SimtWs simt_ws_layout(const Dims& s, size_t es, uint32_t flags) {
   return w;
 }
 
+// Largest dynamic shared memory any SIMT kernel opts in to.  The backward preflight (backward_supported) checks its
+// kernels' sizes against the same constant, so a configuration it accepts cannot fail here at launch time.
+constexpr size_t DYN_SMEM_MAX = 220 * 1024;
+
 // Opt a kernel in to `smem` bytes of dynamic shared memory.  The attribute is read back first and only ever raised:
 // the same kernel template is launched from several translation units, so no TU-local cache may lower it.
 template <typename K>
 static int ensure_dynamic_smem(K kernel, size_t smem) {
-  if (smem > 220 * 1024) return EGNN_ERR_UNSUPPORTED;
+  if (smem > DYN_SMEM_MAX) return EGNN_ERR_UNSUPPORTED;
   if (smem <= 48 * 1024) return EGNN_OK;
   cudaFuncAttributes attr;
   EGNN_CUDA_TRY(cudaFuncGetAttributes(&attr, kernel));

@@ -465,7 +465,15 @@ class EGNN(nn.Module):
             io.pre2_out = None if pre2 is None else pre2.data_ptr()
             if train:     # preflight: configurations the backward kernels cannot run fail HERE, before the forward launches
                 nbb = C.c_size_t()
-                nat.check("egnn_layer_backward_workspace_bytes", lib.egnn_layer_backward_workspace_bytes(C.byref(desc), C.byref(nbb)))
+                rc = lib.egnn_layer_backward_workspace_bytes(C.byref(desc), C.byref(nbb))
+                if rc == nat.ERR_UNSUPPORTED:
+                    raise nat.EgnnNativeError(
+                        "egnn_layer_backward_workspace_bytes", rc,
+                        f"the backward kernels cannot train this layer ({str(kdt).replace('torch.', '')}, dim={self.dim}, "
+                        f"m_dim={self.m_dim}, edge_dim={self.edge_dim}, fourier_features={self.fourier_features}, "
+                        f"{f'k={k} neighbours' if k > 0 else 'dense'}, soft_edges={self.edge_gate is not None}"
+                        f"{'' if rows is None else f', rows {rows[0]}:{rows[1]}'}); see DESIGN.md section 9 'Limits'")
+                nat.check("egnn_layer_backward_workspace_bytes", rc)
             # training keeps the workspace (per-node tables, pooled messages, neighbour lists) for backward
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev) if train else _workspace(dev, ws_bytes, stream_handle)
             nat.check("egnn_layer_forward",

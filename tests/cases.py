@@ -308,6 +308,8 @@ SPECS = {
 # gradient fixtures (25 MB each in float64); they are still checked CUDA-vs-oracle.
 
 # (the global-attention blocks train through PyTorch autograd, not through egnn_layer_backward: no hand-written gradient)
+# knn_k33 / knn_k32_c5 have no committed reference-gradient fixture; tests/test_gpu_grad_shapes.py checks their
+# gradients against the numpy oracle.
 GRAD_SPECS = [n for n in SPECS if not n.startswith("c1_") and not n.startswith("net_global") and n not in {"knn_k33", "knn_k32_c5"}]
 
 

@@ -14,50 +14,6 @@ pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
-def module_grads(case, dtype, device="cuda"):
-    """Run forward + backward of the product module; -> flat {name: float64 numpy gradient}."""
-    mod = util.make_module(case, dtype, device=device)
-    mod.requires_grad_(True)
-    ins = case["inputs"]
-    t = lambda name: util.to_torch(ins.get(name), dtype, device)
-    feats, coors, edges = t("feats"), t("coors"), t("edges")
-    leaves = {"coors": coors.requires_grad_(True)}
-    if feats.is_floating_point():
-        leaves["feats"] = feats.requires_grad_(True)
-    if edges is not None and edges.is_floating_point():
-        leaves["edges"] = edges.requires_grad_(True)
-    gf, gx = (torch.from_numpy(g).to(device=device, dtype=dtype) for g in cases.upstream_grads(case))
-    with torch.enable_grad():
-        if case["kind"] == "network":
-            fo, xo = mod(feats, coors, adj_mat=t("adj_mat"), edges=edges, mask=t("mask"))
-        else:
-            fo, xo = mod(feats, coors, edges, mask=t("mask"), adj_mat=t("adj_mat"))
-        assert fo.requires_grad and xo.requires_grad
-        ((fo * gf).sum() + (xo * gx).sum()).backward()
-    out = {f"in.{k}": v.grad.double().cpu().numpy() for k, v in leaves.items()}
-    for k, p in mod.named_parameters():
-        out[f"p.{k}"] = (torch.zeros_like(p) if p.grad is None else p.grad).double().cpu().numpy()
-    return out
-
-
-def compare(got, want, tol, what):
-    assert set(got) == set(want), (what, sorted(set(got) ^ set(want)))
-    bad = []
-    for k in sorted(want):
-        scale = max(1.0, float(np.abs(want[k]).max()))
-        err = float(np.abs(got[k] - want[k]).max()) / scale
-        if not np.isfinite(got[k]).all() or err > tol:
-            bad.append(f"{k}: rel err {err:.3e}")
-    assert not bad, f"{what}: " + "; ".join(bad)
-
-
-def _tol(case, dtype):
-    if dtype == torch.float64:
-        # CoorsNorm: the oracle (like the reference) carries ~1e-9 of cancellation noise from the 1/eps self pair
-        return 1e-7 if "norm_coors" in str(case["spec"]["cfg"]) else 1e-9
-    return 5e-4
-
-
 def _grad_dtype(name):
     # m_dim = 32 in fp64 exceeds the shared-memory budget of the first backward kernel (EGNN_ERR_UNSUPPORTED)
     return torch.float32 if name == "dense_mdim32" else torch.float64
@@ -70,9 +26,9 @@ GRAD_CASES = cases.GRAD_SPECS + ["c1_dim512_xavier"]
 def test_grads_match_oracle_fp64(name):
     case = cases.build_case(cases.SPECS[name])
     dtype = _grad_dtype(name)
-    got = module_grads(case, dtype)
+    got = util.module_grads(case, dtype)
     want = cases.flatten_grads(cases.run_oracle_grad(case))
-    compare(got, want, _tol(case, dtype), f"{name} vs oracle")
+    util.compare(got, want, util.grad_tol(case, dtype), f"{name} vs oracle")
 
 
 @pytest.mark.parametrize("name", cases.GRAD_SPECS)
@@ -83,18 +39,18 @@ def test_grads_match_reference_fixture_fp64(name):
     case = cases.build_case(cases.SPECS[name])
     assert cases.case_checksum(case) == str(g["checksum"])
     dtype = _grad_dtype(name)
-    got = module_grads(case, dtype)
+    got = util.module_grads(case, dtype)
     want = {k: g[k] for k in g.files if k.startswith(("in.", "p."))}
-    compare(got, want, _tol(case, dtype), f"{name} vs reference autograd")
+    util.compare(got, want, util.grad_tol(case, dtype), f"{name} vs reference autograd")
 
 
 @pytest.mark.parametrize("name", ["dense_xavier", "dense_everything", "knn_edges_mask", "adj_sparse_random",
                                   "net_c3_xavier", "net_c5_xavier", "dense_mdim32"])
 def test_grads_fp32(name):
     case = cases.build_case(cases.SPECS[name])
-    got = module_grads(case, torch.float32)
+    got = util.module_grads(case, torch.float32)
     want = cases.flatten_grads(cases.run_oracle_grad(case))
-    compare(got, want, _tol(case, torch.float32), f"{name} fp32 vs oracle")
+    util.compare(got, want, util.grad_tol(case, torch.float32), f"{name} fp32 vs oracle")
 
 
 @pytest.mark.parametrize("name", ["dense_everything", "dense_edges", "c1_dim512_xavier", "net_dense_feats", "knn_edges_mask",
@@ -104,18 +60,18 @@ def test_grads_with_recompute_instead_of_saved_pair_activations(name, monkeypatc
     recomputes them with the register-tiled forward kernel -- both routes must give the same gradients."""
     monkeypatch.setenv("EGNN_B200_SAVE_PAIR_MB", "0")
     case = cases.build_case(cases.SPECS[name])
-    got = module_grads(case, torch.float64)
+    got = util.module_grads(case, torch.float64)
     want = cases.flatten_grads(cases.run_oracle_grad(case))
-    compare(got, want, _tol(case, torch.float64), f"{name} (recompute) vs oracle")
+    util.compare(got, want, util.grad_tol(case, torch.float64), f"{name} (recompute) vs oracle")
 
 
 def test_cpu_tensors_and_bf16_modules_train_through_the_gpu_kernels():
     """CPU fp64 tensors (how the reference's tests call the layer) get CPU gradients; a bf16 module trains through
     the fp32 kernels and returns bf16 gradients."""
     case = cases.build_case(cases.SPECS["dense_edges"])
-    got = module_grads(case, torch.float64, device="cpu")
+    got = util.module_grads(case, torch.float64, device="cpu")
     want = cases.flatten_grads(cases.run_oracle_grad(case))
-    compare(got, want, 1e-9, "cpu staging")
+    util.compare(got, want, 1e-9, "cpu staging")
     mod = util.make_module(case, torch.bfloat16).requires_grad_(True)
     ins = case["inputs"]
     f = util.to_torch(ins["feats"], torch.bfloat16, "cuda").requires_grad_(True)
