@@ -6,7 +6,7 @@
 //     next[i] = OR_{j : adj[i][j]} adj[j]            (boolean matrix square)
 //     newly   = next XOR adj   -> labels := degree   (:426-427: "(next.float() - adj.float()).bool()")
 //     adj     = next                                 (:428; the EXPANDED matrix is squared again)
-#include "common.cuh"
+#include "launch.cuh"
 
 namespace egnn {
 
@@ -106,21 +106,15 @@ extern "C" int egnn_adj_expand(int32_t B, int32_t N, int32_t num_degrees, const 
   uint32_t* b0 = static_cast<uint32_t*>(workspace);
   uint32_t* b1 = reinterpret_cast<uint32_t*>(static_cast<char*>(workspace) + need / 2);
   const size_t warps = (size_t)B * N * W;
-  adj_pack_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, st>>>(adj_in, adj_batched, B, N, W, b0, labels_out);
-  EGNN_LAUNCH_CHECK();
+  EGNN_TRY(launch(adj_pack_kernel, (unsigned)((warps * 32 + 255) / 256), 256, 0, st, adj_in, adj_batched, B, N, W, b0, labels_out));
   const size_t nb_smem = (size_t)N * sizeof(int);
   if (nb_smem > 200 * 1024) return EGNN_ERR_UNSUPPORTED;
-  if (num_degrees > 1)
-    EGNN_CUDA_TRY(cudaFuncSetAttribute(adj_square_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)nb_smem));
   for (int degree = 2; degree <= num_degrees; ++degree) {
-    adj_square_kernel<<<B * N, 128, nb_smem, st>>>(b0, b1, labels_out, N, W, degree);
-    EGNN_LAUNCH_CHECK();
+    EGNN_TRY(launch(adj_square_kernel, B * N, 128, nb_smem, st, b0, b1, labels_out, N, W, degree));
     uint32_t* t = b0; b0 = b1; b1 = t;
   }
   if (max_row_sum) EGNN_CUDA_TRY(cudaMemsetAsync(max_row_sum, 0, sizeof(int32_t), st));
-  adj_unpack_kernel<<<(unsigned)(((size_t)B * N * 32 + 255) / 256), 256, 0, st>>>(b0, B, N, W, adj_out, max_row_sum);
-  EGNN_LAUNCH_CHECK();
-  return EGNN_OK;
+  return launch(adj_unpack_kernel, (unsigned)(((size_t)B * N * 32 + 255) / 256), 256, 0, st, b0, B, N, W, adj_out, max_row_sum);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -155,18 +149,13 @@ extern "C" int egnn_embed_nodes(int32_t dtype, int32_t B, int32_t N, int32_t dim
                                 const void* token_emb, const void* pos_emb, void* out, void* stream) {
   if (!tokens || !token_emb || !out) return EGNN_ERR_NULL;
   if (B <= 0 || N <= 0 || dim <= 0 || num_tokens <= 0) return EGNN_ERR_SHAPE;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
   const unsigned grid = (unsigned)(((size_t)B * N * 32 + 255) / 256);
-  if (dtype == EGNN_DTYPE_F64)
-    egnn::embed_nodes_kernel<double><<<grid, 256, 0, st>>>(tokens, static_cast<const double*>(token_emb), static_cast<const double*>(pos_emb),
-                                                           static_cast<double*>(out), B, N, dim, num_tokens);
-  else if (dtype == EGNN_DTYPE_F32)
-    egnn::embed_nodes_kernel<float><<<grid, 256, 0, st>>>(tokens, static_cast<const float*>(token_emb), static_cast<const float*>(pos_emb),
-                                                          static_cast<float*>(out), B, N, dim, num_tokens);
-  else
-    egnn::embed_nodes_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(tokens, static_cast<const __nv_bfloat16*>(token_emb),
-                                                                  static_cast<const __nv_bfloat16*>(pos_emb),
-                                                                  static_cast<__nv_bfloat16*>(out), B, N, dim, num_tokens);
-  EGNN_LAUNCH_CHECK();
-  return EGNN_OK;
+  auto run = [&](auto elem) {
+    using T = decltype(elem);
+    return egnn::launch(egnn::embed_nodes_kernel<T>, grid, 256, 0, static_cast<cudaStream_t>(stream), tokens,
+                        static_cast<const T*>(token_emb), static_cast<const T*>(pos_emb), static_cast<T*>(out), B, N, dim, num_tokens);
+  };
+  if (dtype == EGNN_DTYPE_F64) return run(double{});
+  if (dtype == EGNN_DTYPE_F32) return run(float{});
+  return run(__nv_bfloat16{});
 }

@@ -24,12 +24,16 @@ namespace egnn {
     if (_r != EGNN_OK) return _r;                                   \
   } while (0)
 
-// Launch check that does not synchronise: catches bad configurations at enqueue time.
-#define EGNN_LAUNCH_CHECK() EGNN_CUDA_TRY(cudaPeekAtLastError())
-
 __host__ __device__ inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 __host__ __device__ inline size_t round_up(size_t a, size_t b) { return (a + b - 1) / b * b; }
 __host__ __device__ inline int round_up_i(int a, int b) { return (a + b - 1) / b * b; }
+
+// Lays blocks out back to back in one buffer: take() returns the offset of the next block, and each block's size is
+// rounded up to `align` so the one after it starts aligned.
+struct BumpAlloc {
+  size_t total = 0;
+  size_t take(size_t n, size_t align = 256) { const size_t r = total; total += round_up(n, align); return r; }
+};
 
 // ------------------------------------------------------------------ derived sizes
 struct Dims {
@@ -188,16 +192,15 @@ struct SimtPackLayout {
 inline SimtPackLayout simt_pack_layout(const Dims& s) {
   SimtPackLayout L;
   L.MP = s.m <= 16 ? 16 : 32;
-  size_t o = 0;
-  auto take = [&](size_t n) { size_t r = o; o += round_up(n, 4); return r; };
-  L.w2t = take((size_t)s.Hp * L.MP);
-  L.wq = take((size_t)s.Q * s.Hp);
-  L.tab = take((size_t)(s.label_dim > 0 ? s.num_labels : 0) * s.Hp);
-  L.w3 = take((size_t)4 * s.m * L.MP);
-  L.b3 = take((size_t)4 * s.m);
-  L.w4 = take((size_t)4 * s.m);
-  L.misc = take((size_t)2 * L.MP + 4);
-  L.total = o;
+  BumpAlloc o;
+  L.w2t = o.take((size_t)s.Hp * L.MP, 4);
+  L.wq = o.take((size_t)s.Q * s.Hp, 4);
+  L.tab = o.take((size_t)(s.label_dim > 0 ? s.num_labels : 0) * s.Hp, 4);
+  L.w3 = o.take((size_t)4 * s.m * L.MP, 4);
+  L.b3 = o.take((size_t)4 * s.m, 4);
+  L.w4 = o.take((size_t)4 * s.m, 4);
+  L.misc = o.take((size_t)2 * L.MP + 4, 4);
+  L.total = o.total;
   return L;
 }
 

@@ -3,52 +3,31 @@
 #include "common.cuh"
 #include "simt_kernels.cuh"
 #include "fast_path.h"
-#include "profile.h"
+#include "knn_select.h"
 #include "simt_host.cuh"
 #include "small_node.cuh"
 #include <algorithm>
 
 namespace egnn {
 
-int knn_select_dispatch(int32_t dtype, int B, int N, int C, int k, const void* coors, const uint8_t* mask,
-                        const uint8_t* adj, int adj_batched, double valid_radius, int32_t* out_idx,
-                        uint8_t* out_ok, cudaStream_t st);
-int adj_neighbors_dispatch(int B, int N, int k, const uint8_t* adj, int adj_batched, int32_t* out_idx, uint8_t* out_ok,
-                           cudaStream_t st);
-
 template <typename T, int MP, bool KNN>
 static int launch_pair(const PairArgs<T>& a, cudaStream_t st) {
-  const size_t smem = pair_smem_bytes<T>(a.s, a.L, KNN);
-  EGNN_TRY(ensure_dynamic_smem(pair_kernel<T, MP, KNN>, smem));
-  const int TI = PAIR_THREADS / a.TS;
-  dim3 grid(ceil_div(a.s.row1 - a.s.row0, TI), a.s.B);
-  pair_kernel<T, MP, KNN><<<grid, PAIR_THREADS, smem, st>>>(a);
-  EGNN_LAUNCH_CHECK();
-  count_launch();
-  return EGNN_OK;
+  dim3 grid(ceil_div(a.s.row1 - a.s.row0, PAIR_THREADS / a.TS), a.s.B);
+  return launch(pair_kernel<T, MP, KNN>, grid, PAIR_THREADS, pair_smem_bytes<T>(a.s, a.L, KNN), st, a);
 }
 
 template <typename T, int MP, int PP>
 static int launch_pair_tiled(const PairArgs<T>& a, cudaStream_t st) {
   const size_t smem = pair_tiled_smem_bytes<T>(a.s, a.L, PP);
-  EGNN_TRY(ensure_dynamic_smem(pair_dense_tiled_kernel<T, MP, PP>, smem));
   dim3 grid(ceil_div(a.s.row1 - a.s.row0, 4 * PP), a.s.B);
   if (a.hsplit > 1) {
     PairArgs<T> a1 = a, a2 = a;
     a1.phase = 1; a2.phase = 2;
     a1.pre2_out = nullptr;                            // partial sums; phase 2 holds the full ones
-    dim3 g1(grid.x, grid.y, a.hsplit);
-    pair_dense_tiled_kernel<T, MP, PP><<<g1, PAIR_THREADS, smem, st>>>(a1);
-    EGNN_LAUNCH_CHECK();
-    pair_dense_tiled_kernel<T, MP, PP><<<grid, PAIR_THREADS, smem, st>>>(a2);
-    EGNN_LAUNCH_CHECK();
-    count_launch(2);
-    return EGNN_OK;
+    EGNN_TRY(launch(pair_dense_tiled_kernel<T, MP, PP>, dim3(grid.x, grid.y, a.hsplit), PAIR_THREADS, smem, st, a1));
+    return launch(pair_dense_tiled_kernel<T, MP, PP>, grid, PAIR_THREADS, smem, st, a2);
   }
-  pair_dense_tiled_kernel<T, MP, PP><<<grid, PAIR_THREADS, smem, st>>>(a);
-  EGNN_LAUNCH_CHECK();
-  count_launch();
-  return EGNN_OK;
+  return launch(pair_dense_tiled_kernel<T, MP, PP>, grid, PAIR_THREADS, smem, st, a);
 }
 
 template <typename T>
@@ -71,19 +50,7 @@ static int simt_forward(const EgnnLayerDesc& d, const EgnnLayerWeights& w, const
   const RowMap ident{s.N, s.N, 0};
 
   // 1. neighbour lists (egnn_pytorch.py:237-260)
-  if (s.k > 0 && io.nbr_idx) {                       // edge-list mode: the caller's lists, no ranking
-    nbr_idx = const_cast<int32_t*>(io.nbr_idx);
-    nbr_ok = nullptr;
-  } else if (s.k > 0) {
-    StageTimer tm(st, STAGE_SELECT);
-    count_launch();
-    const double vr = (d.flags & EGNN_FLAG_ONLY_SPARSE) ? 0.0 : d.valid_radius;     // :250
-    if ((d.flags & EGNN_FLAG_ONLY_SPARSE) && io.mask && io.adj)      // every slot top-k could add is masked out: row scan
-      EGNN_TRY(adj_neighbors_dispatch(s.B, s.N, s.k, io.adj, (d.flags & EGNN_FLAG_ADJ_BATCHED) ? 1 : 0, nbr_idx, nbr_ok, st));
-    else
-      EGNN_TRY(knn_select_dispatch(d.dtype, s.B, s.N, s.C, s.k, io.coors, io.mask, io.adj,
-                                   (d.flags & EGNN_FLAG_ADJ_BATCHED) ? 1 : 0, vr, nbr_idx, nbr_ok, st));
-  }
+  if (s.k > 0) EGNN_TRY(select_neighbours(d, s, io, d.dtype, nbr_idx, nbr_ok, st));
   // 2. per-node tables  A = h W1[:, :dim]^T + b1,  B = h W1[:, dim:2dim]^T   (split of :287's Linear-1)
   {
     StageTimer tm(st, STAGE_NODE_PRE);
@@ -91,11 +58,10 @@ static int simt_forward(const EgnnLayerDesc& d, const EgnnLayerWeights& w, const
       TablesSmallSimtArgs<T> t;
       t.feats = feats; t.W1 = W1; t.b1 = static_cast<const T*>(w.edge_b1); t.P = P;
       t.M = s.M; t.dim = s.dim; t.H = s.H; t.Hp = s.Hp; t.E = s.E;
-      const size_t smem = tables_small_simt_smem<T>(s.dim, s.Hp);
-      EGNN_TRY(ensure_dynamic_smem(tables_small_simt_kernel<T>, smem));
-      tables_small_simt_kernel<T><<<std::min(ceil_div(s.M, SN_WARPS), 4 * small_node_sms()), SN_WARPS * 32, smem, st>>>(t);
-      EGNN_LAUNCH_CHECK();
-      count_launch();
+      int sms = 0;
+      EGNN_TRY(device_sm_count(&sms));
+      EGNN_TRY(launch(tables_small_simt_kernel<T>, std::min(ceil_div(s.M, SN_WARPS), 4 * sms), SN_WARPS * 32,
+                      tables_small_simt_smem<T>(s.dim, s.Hp), st, t));
     } else {
       EGNN_TRY((launch_gemm<T, 0, false>(feats, s.dim, W1, s.E, static_cast<const T*>(w.edge_b1), nullptr, 0, P,
                                           2 * s.Hp, s.M, s.H, s.Hp, s.dim, ident, st)));
@@ -155,17 +121,13 @@ static int simt_forward(const EgnnLayerDesc& d, const EgnnLayerWeights& w, const
     n.out = static_cast<T*>(io.feats_out);
     n.B = s.B; n.N = s.N; n.dim = s.dim; n.m = s.m; n.row0 = s.row0; n.row1 = s.row1;
     n.do_norm = (d.flags & EGNN_FLAG_NORM_FEATS) ? 1 : 0;
-    const size_t smem = node_small_simt_smem<T>(s.dim, s.m);
-    EGNN_TRY(ensure_dynamic_smem(node_update_small_simt_kernel<T>, smem));
-    node_update_small_simt_kernel<T><<<std::min(ceil_div(Mr, SN_WARPS), 4 * small_node_sms()), SN_WARPS * 32, smem, st>>>(n);
-    EGNN_LAUNCH_CHECK();
-    count_launch();
+    int sms = 0;
+    EGNN_TRY(device_sm_count(&sms));
+    EGNN_TRY(launch(node_update_small_simt_kernel<T>, std::min(ceil_div(Mr, SN_WARPS), 4 * sms), SN_WARPS * 32,
+                    node_small_simt_smem<T>(s.dim, s.m), st, n));
   } else if (uf) {
-    ln_concat_kernel<T><<<ceil_div(Mr * 32, 256), 256, 0, st>>>(
-        feats, static_cast<const T*>(w.norm_g), static_cast<const T*>(w.norm_b), node_in, s.dim + s.m, s.dim, Mr,
-        map, (d.flags & EGNN_FLAG_NORM_FEATS) ? 1 : 0);
-    EGNN_LAUNCH_CHECK();
-    count_launch();
+    EGNN_TRY(launch(ln_concat_kernel<T>, ceil_div(Mr * 32, 256), 256, 0, st, feats, static_cast<const T*>(w.norm_g),
+                    static_cast<const T*>(w.norm_b), node_in, s.dim + s.m, s.dim, Mr, map, (d.flags & EGNN_FLAG_NORM_FEATS) ? 1 : 0));
     EGNN_TRY((launch_gemm<T, 1, false>(node_in, s.dim + s.m, static_cast<const T*>(w.node_w1), s.dim + s.m,
                                        static_cast<const T*>(w.node_b1), nullptr, 0, h1, 2 * s.dim, Mr, 2 * s.dim,
                                        2 * s.dim, s.dim + s.m, map, st, make_drop(d.dropout_p, d.dropout_seed))));
@@ -223,12 +185,8 @@ extern "C" int egnn_layer_pack_weights(const EgnnLayerDesc* desc, const EgnnLaye
   const Dims s = make_dims(*desc);
   if (desc->dtype == EGNN_DTYPE_BF16) return fast_pack_weights(*desc, *w, packed, packed_bytes, st);
   const SimtPackLayout L = simt_pack_layout(s);
-  if (desc->dtype == EGNN_DTYPE_F64)
-    simt_pack_kernel<double><<<148, 256, 0, st>>>(s, L, *w, desc->flags, static_cast<double*>(packed));
-  else
-    simt_pack_kernel<float><<<148, 256, 0, st>>>(s, L, *w, desc->flags, static_cast<float*>(packed));
-  EGNN_LAUNCH_CHECK();
-  return EGNN_OK;
+  if (desc->dtype == EGNN_DTYPE_F64) return launch(simt_pack_kernel<double>, 148, 256, 0, st, s, L, *w, desc->flags, static_cast<double*>(packed));
+  return launch(simt_pack_kernel<float>, 148, 256, 0, st, s, L, *w, desc->flags, static_cast<float*>(packed));
 }
 
 extern "C" int egnn_layer_workspace_bytes(const EgnnLayerDesc* desc, size_t* out_bytes) {

@@ -15,19 +15,18 @@ struct BwdWs {
 
 inline BwdWs bwd_ws_layout(const Dims& s, const SimtPackLayout& L, size_t es, uint32_t flags) {
   BwdWs w;
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t r = o; o += round_up(bytes, 256); return r; };
+  BumpAlloc o;
   const size_t J = s.k > 0 ? s.k : s.N;
   const bool uf = flags & EGNN_FLAG_UPDATE_FEATS;
-  w.gP = take((size_t)s.M * 2 * s.Hp * es);
-  w.gpk = take(L.total * es);
-  w.rec = take((size_t)s.M * J * rec_layout(s, L.MP).R * es);
-  w.pre2 = take(s.k == 0 ? (size_t)s.M * s.N * L.MP * es : 0);
-  w.h1pre = take(uf ? (size_t)s.M * 2 * s.dim * es : 0);
-  w.ga = take(uf ? (size_t)s.M * 2 * s.dim * es : 0);
-  w.g_node_in = take(uf ? (size_t)s.M * (s.dim + s.m) * es : 0);
-  w.gyx = take((uf && (flags & EGNN_FLAG_NORM_FEATS)) ? (size_t)s.M * s.dim * es : 0);
-  w.total = o;
+  w.gP = o.take((size_t)s.M * 2 * s.Hp * es);
+  w.gpk = o.take(L.total * es);
+  w.rec = o.take((size_t)s.M * J * rec_layout(s, L.MP).R * es);
+  w.pre2 = o.take(s.k == 0 ? (size_t)s.M * s.N * L.MP * es : 0);
+  w.h1pre = o.take(uf ? (size_t)s.M * 2 * s.dim * es : 0);
+  w.ga = o.take(uf ? (size_t)s.M * 2 * s.dim * es : 0);
+  w.g_node_in = o.take(uf ? (size_t)s.M * (s.dim + s.m) * es : 0);
+  w.gyx = o.take((uf && (flags & EGNN_FLAG_NORM_FEATS)) ? (size_t)s.M * s.dim * es : 0);
+  w.total = o.total;
   return w;
 }
 
@@ -49,7 +48,7 @@ inline int backward_supported(const EgnnLayerDesc& d) {
   if (d.label_dim > 0 && d.num_labels > BW2_MAXLAB) return EGNN_ERR_UNSUPPORTED;
   const Dims s = make_dims(d);
   const size_t smem = d.dtype == EGNN_DTYPE_F64 ? backward_smem_bytes<double>(s, d.flags) : backward_smem_bytes<float>(s, d.flags);
-  if (smem > DYN_SMEM_MAX) return EGNN_ERR_UNSUPPORTED;     // ensure_dynamic_smem would refuse it at launch
+  if (smem > DYN_SMEM_MAX) return EGNN_ERR_UNSUPPORTED;     // launch() would refuse it
   return EGNN_OK;
 }
 
@@ -63,23 +62,16 @@ static int launch_gemm_acc(const T* A, long ars, long aks, const T* B, long bks,
   splits = std::min(splits, 65535);
   const int kper = round_up_i(ceil_div(K, splits), 16);
   splits = ceil_div(K, kper);
-  dim3 grid(ceil_div(Nc, 64), ceil_div(Mr, 64), splits);
-  gemm_acc_kernel<T><<<grid, 256, 0, st>>>(A, ars, aks, B, bks, bcs, C, ldc, Mr, Nc, K, kper);
-  EGNN_LAUNCH_CHECK();
-  return EGNN_OK;
+  return launch(gemm_acc_kernel<T>, dim3(ceil_div(Nc, 64), ceil_div(Mr, 64), splits), 256, 0, st, A, ars, aks, B, bks, bcs, C, ldc, Mr, Nc,
+                K, kper);
 }
 
 template <typename T>
 static int launch_colsum(const T* X, long ld, int rows, int cols, T* out, cudaStream_t st) {
   if (rows <= 0 || cols <= 0) return EGNN_OK;
   dim3 grid(ceil_div(cols, 32), std::max(1, std::min(64, ceil_div(rows, 64))));
-  colsum_acc_kernel<T><<<grid, dim3(32, 8), 0, st>>>(X, ld, rows, cols, out);
-  EGNN_LAUNCH_CHECK();
-  return EGNN_OK;
+  return launch(colsum_acc_kernel<T>, grid, dim3(32, 8), 0, st, X, ld, rows, cols, out);
 }
-
-template <typename K>
-static int opt_in_smem(K kernel, size_t smem) { return ensure_dynamic_smem(kernel, smem); }
 
 // Dense: W2 silu(pre1) for every pair with the register-tiled forward kernel (its split-H "phase 1" stores exactly
 // that); returns EGNN_ERR_UNSUPPORTED when its shared memory does not fit, and bwd1 then recomputes by itself.
@@ -93,12 +85,8 @@ static int launch_tiled_recompute(const BwdArgs<T>& a, T* pre2, cudaStream_t st)
   f.hpart = pre2; f.hsplit = 1; f.phase = 1;
   f.pre2_out = nullptr;
   f.drop = a.drop;                                    // the recompute must draw the forward's masks
-  const size_t smem = pair_tiled_smem_bytes<T>(a.s, a.L, PP);
-  EGNN_TRY(opt_in_smem(pair_dense_tiled_kernel<T, MP, PP>, smem));
-  dim3 grid(ceil_div(a.s.N, 4 * PP), a.s.B, 1);
-  pair_dense_tiled_kernel<T, MP, PP><<<grid, PAIR_THREADS, smem, st>>>(f);
-  EGNN_LAUNCH_CHECK();
-  return EGNN_OK;
+  return launch(pair_dense_tiled_kernel<T, MP, PP>, dim3(ceil_div(a.s.N, 4 * PP), a.s.B, 1), PAIR_THREADS,
+                pair_tiled_smem_bytes<T>(a.s, a.L, PP), st, f);
 }
 
 template <typename T, int MP, bool KNN>
@@ -112,65 +100,22 @@ static int launch_pair_bwd(BwdArgs<T>& a, bool saved_pre2, cudaStream_t st) {
     else EGNN_TRY(rc);
     }
   }
-  const size_t smem1 = bwd1_smem_bytes<T>(s, a.L, KNN, (a.flags & EGNN_FLAG_SOFT_EDGES) != 0);
-  EGNN_TRY(opt_in_smem(pair_bwd1_kernel<T, MP, KNN>, smem1));
   const int TI = PAIR_THREADS / a.TS;
   dim3 g1(ceil_div(s.N, TI), s.B);
-  pair_bwd1_kernel<T, MP, KNN><<<g1, PAIR_THREADS, smem1, st>>>(a);
-  EGNN_LAUNCH_CHECK();
+  EGNN_TRY(launch(pair_bwd1_kernel<T, MP, KNN>, g1, PAIR_THREADS,
+                  bwd1_smem_bytes<T>(s, a.L, KNN, (a.flags & EGNN_FLAG_SOFT_EDGES) != 0), st, a));
+  const bool q1 = s.Q == 1 && s.label_dim == 0, drop = a.drop.thr != 0;
   if constexpr (KNN) {
-    const size_t smem2 = bwd2_knn_smem_bytes<T>(s, a.rl.R);
-    dim3 g2(ceil_div(s.N, a.TI2), ceil_div(s.Hp, BW2_TH), s.B);
-    if (s.Q == 1 && s.label_dim == 0) {
-      if (a.drop.thr) {
-        EGNN_TRY(opt_in_smem(pair_bwd2_knn_kernel<T, MP, 1, true>, smem2));
-        pair_bwd2_knn_kernel<T, MP, 1, true><<<g2, BW2_TH, smem2, st>>>(a);
-      } else {
-        EGNN_TRY(opt_in_smem(pair_bwd2_knn_kernel<T, MP, 1, false>, smem2));
-        pair_bwd2_knn_kernel<T, MP, 1, false><<<g2, BW2_TH, smem2, st>>>(a);
-      }
-    } else if (s.Q <= 8) {
-      if (a.drop.thr) {
-        EGNN_TRY(opt_in_smem(pair_bwd2_knn_kernel<T, MP, 8, true>, smem2));
-        pair_bwd2_knn_kernel<T, MP, 8, true><<<g2, BW2_TH, smem2, st>>>(a);
-      } else {
-        EGNN_TRY(opt_in_smem(pair_bwd2_knn_kernel<T, MP, 8, false>, smem2));
-        pair_bwd2_knn_kernel<T, MP, 8, false><<<g2, BW2_TH, smem2, st>>>(a);
-      }
-    } else {
-      if (a.drop.thr) {
-        EGNN_TRY(opt_in_smem(pair_bwd2_knn_kernel<T, MP, 0, true>, smem2));
-        pair_bwd2_knn_kernel<T, MP, 0, true><<<g2, BW2_TH, smem2, st>>>(a);
-      } else {
-        EGNN_TRY(opt_in_smem(pair_bwd2_knn_kernel<T, MP, 0, false>, smem2));
-        pair_bwd2_knn_kernel<T, MP, 0, false><<<g2, BW2_TH, smem2, st>>>(a);
-      }
-    }
+    auto bwd2 = q1 ? (drop ? pair_bwd2_knn_kernel<T, MP, 1, true> : pair_bwd2_knn_kernel<T, MP, 1, false>)
+              : s.Q <= 8 ? (drop ? pair_bwd2_knn_kernel<T, MP, 8, true> : pair_bwd2_knn_kernel<T, MP, 8, false>)
+                         : (drop ? pair_bwd2_knn_kernel<T, MP, 0, true> : pair_bwd2_knn_kernel<T, MP, 0, false>);
+    EGNN_TRY(launch(bwd2, dim3(ceil_div(s.N, a.TI2), ceil_div(s.Hp, BW2_TH), s.B), BW2_TH, bwd2_knn_smem_bytes<T>(s, a.rl.R), st, a));
   } else {
-    const size_t smem2 = bwd2_dense_smem_bytes<T>(s, a.rl.R);
-    dim3 g2(ceil_div(s.N, BW2_ROWS), ceil_div(s.Hp, BW2_TH), s.B);
-    if (s.Q == 1 && s.label_dim == 0) {
-      if (a.drop.thr) {
-        EGNN_TRY(opt_in_smem(pair_bwd2_dense_kernel<T, MP, 1, true>, smem2));
-        pair_bwd2_dense_kernel<T, MP, 1, true><<<g2, BW2_TH, smem2, st>>>(a);
-      } else {
-        EGNN_TRY(opt_in_smem(pair_bwd2_dense_kernel<T, MP, 1, false>, smem2));
-        pair_bwd2_dense_kernel<T, MP, 1, false><<<g2, BW2_TH, smem2, st>>>(a);
-      }
-    } else {
-      if (a.drop.thr) {
-        EGNN_TRY(opt_in_smem(pair_bwd2_dense_kernel<T, MP, 0, true>, smem2));
-        pair_bwd2_dense_kernel<T, MP, 0, true><<<g2, BW2_TH, smem2, st>>>(a);
-      } else {
-        EGNN_TRY(opt_in_smem(pair_bwd2_dense_kernel<T, MP, 0, false>, smem2));
-        pair_bwd2_dense_kernel<T, MP, 0, false><<<g2, BW2_TH, smem2, st>>>(a);
-      }
-    }
+    auto bwd2 = q1 ? (drop ? pair_bwd2_dense_kernel<T, MP, 1, true> : pair_bwd2_dense_kernel<T, MP, 1, false>)
+                   : (drop ? pair_bwd2_dense_kernel<T, MP, 0, true> : pair_bwd2_dense_kernel<T, MP, 0, false>);
+    EGNN_TRY(launch(bwd2, dim3(ceil_div(s.N, BW2_ROWS), ceil_div(s.Hp, BW2_TH), s.B), BW2_TH, bwd2_dense_smem_bytes<T>(s, a.rl.R), st, a));
   }
-  EGNN_LAUNCH_CHECK();
-  pair_bwd3_kernel<T, KNN><<<g1, PAIR_THREADS, 0, st>>>(a);
-  EGNN_LAUNCH_CHECK();
-  return EGNN_OK;
+  return launch(pair_bwd3_kernel<T, KNN>, g1, PAIR_THREADS, 0, st, a);
 }
 
 template <typename T>
@@ -251,16 +196,14 @@ int simt_backward(const EgnnLayerDesc& d, const EgnnLayerWeights& w, const void*
     EGNN_TRY(launch_gemm_acc<T>(go, 1, dim, h1, d2, 1, static_cast<T*>(gr.w.node_w2), d2, dim, d2, M, st));
     EGNN_TRY(launch_colsum<T>(go, dim, M, dim, static_cast<T*>(gr.w.node_b2), st));
     EGNN_TRY(launch_gemm_acc<T>(go, dim, 1, Wn2, d2, 1, ga, d2, M, d2, dim, st));
-    dsilu_mul_kernel<T><<<(int)std::min<size_t>(2048, ((size_t)M * d2 + 255) / 256), 256, 0, st>>>(ga, h1pre, (size_t)M * d2,
-                                                                                                     make_drop(d.dropout_p, d.dropout_seed));
-    EGNN_LAUNCH_CHECK();
+    EGNN_TRY(launch(dsilu_mul_kernel<T>, (int)std::min<size_t>(2048, ((size_t)M * d2 + 255) / 256), 256, 0, st, ga, h1pre,
+                    (size_t)M * d2, make_drop(d.dropout_p, d.dropout_seed)));
     // dWn1[k][c] = sum_r gh1[r][k] node_in[r][c];  db1 = colsum(gh1);  g_node_in = gh1 Wn1
     EGNN_TRY(launch_gemm_acc<T>(ga, 1, d2, node_in, dn, 1, static_cast<T*>(gr.w.node_w1), dn, d2, dn, M, st));
     EGNN_TRY(launch_colsum<T>(ga, d2, M, d2, static_cast<T*>(gr.w.node_b1), st));
     EGNN_TRY(launch_gemm_acc<T>(ga, d2, 1, Wn1, dn, 1, g_node_in, dn, M, dn, d2, st));
-    ln_bwd_kernel<T><<<ceil_div(M * 32, 256), 256, 0, st>>>(feats, static_cast<const T*>(w.norm_g), g_node_in, dn,
-                                                            g_feats, gyx, dim, M, nf ? 1 : 0);
-    EGNN_LAUNCH_CHECK();
+    EGNN_TRY(launch(ln_bwd_kernel<T>, ceil_div(M * 32, 256), 256, 0, st, feats, static_cast<const T*>(w.norm_g), g_node_in, dn,
+                    g_feats, gyx, dim, M, nf ? 1 : 0));
     if (nf) {
       EGNN_TRY(launch_colsum<T>(gyx, dim, M, dim, static_cast<T*>(gr.w.norm_g), st));
       EGNN_TRY(launch_colsum<T>(g_node_in, dn, M, dim, static_cast<T*>(gr.w.norm_b), st));
@@ -307,10 +250,8 @@ int simt_backward(const EgnnLayerDesc& d, const EgnnLayerWeights& w, const void*
   EGNN_TRY(launch_gemm_acc<T>(gP + s.Hp, 1, ldP, feats, dim, 1, gW1 + dim, s.E, s.H, dim, M, st));      // dW1_j = gB^T h
   EGNN_TRY(launch_colsum<T>(gP, ldP, M, s.H, static_cast<T*>(gr.w.edge_b1), st));                       // db1
 
-  unpack_grads_kernel<T><<<148, 256, 0, st>>>(s, L, d.flags, gpk, W1, static_cast<const T*>(w.label_emb), gr.w);
-  EGNN_LAUNCH_CHECK();
   (void)uc; (void)h1;
-  return EGNN_OK;
+  return launch(unpack_grads_kernel<T>, 148, 256, 0, st, s, L, d.flags, gpk, W1, static_cast<const T*>(w.label_emb), gr.w);
 }
 
 }  // namespace egnn

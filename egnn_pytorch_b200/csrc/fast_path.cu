@@ -4,22 +4,15 @@
 // Option sets the tensor-core kernels do not cover return EGNN_ERR_UNSUPPORTED; the binding then runs
 // the fp32 SIMT kernels (never a CPU path).
 #include <stdlib.h>
-#include <mutex>
 #include "fast_path.h"
-#include "profile.h"
+#include "knn_select.h"
+#include "launch.cuh"
 #include "tc_gemm.cuh"
 #include "tc_pair.cuh"
 #include "tc_knn.cuh"
 #include "small_node.cuh"
 
 namespace egnn {
-
-int knn_select_dispatch(int32_t dtype, int B, int N, int C, int k, const void* coors, const uint8_t* mask,
-                        const uint8_t* adj, int adj_batched, double valid_radius, int32_t* out_idx,
-                        uint8_t* out_ok, cudaStream_t st);
-int adj_neighbors_dispatch(int B, int N, int k, const uint8_t* adj, int adj_batched, int32_t* out_idx, uint8_t* out_ok,
-                           cudaStream_t st);
-
 namespace {
 
 struct FastDims {
@@ -58,22 +51,21 @@ bool pair_is_lean(const FastDims& f) { return f.s.C == 3 && f.QT == 1; }
 
 FastPack fast_pack_layout(const FastDims& f) {
   FastPack p;
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t r = o; o += round_up(bytes, 256); return r; };
+  BumpAlloc o;
   const int d = f.s.dim;
-  p.w1i = take((size_t)f.Hp * d * 2);
-  p.w1j = take((size_t)f.Hp * d * 2);
-  p.b1 = take((size_t)f.Hp * 4);
-  p.wq = take((size_t)f.QR * f.Hp * 4);
-  p.w2p = take((size_t)f.Hp * 32);
-  p.epi = take((size_t)TP_EPI_FLOATS * 4);
-  p.wn1 = take((size_t)2 * d * f.Kn * 2);
-  p.bn1 = take((size_t)2 * d * 4);
-  p.wn2 = take((size_t)d * 2 * d * 2);
-  p.bn2 = take((size_t)d * 4);
-  p.lng = take((size_t)d * 4);
-  p.lnb = take((size_t)d * 4);
-  p.total = o;
+  p.w1i = o.take((size_t)f.Hp * d * 2);
+  p.w1j = o.take((size_t)f.Hp * d * 2);
+  p.b1 = o.take((size_t)f.Hp * 4);
+  p.wq = o.take((size_t)f.QR * f.Hp * 4);
+  p.w2p = o.take((size_t)f.Hp * 32);
+  p.epi = o.take((size_t)TP_EPI_FLOATS * 4);
+  p.wn1 = o.take((size_t)2 * d * f.Kn * 2);
+  p.bn1 = o.take((size_t)2 * d * 4);
+  p.wn2 = o.take((size_t)d * 2 * d * 2);
+  p.bn2 = o.take((size_t)d * 4);
+  p.lng = o.take((size_t)d * 4);
+  p.lnb = o.take((size_t)d * 4);
+  p.total = o.total;
   return p;
 }
 
@@ -85,12 +77,12 @@ int fast_supported(const EgnnLayerDesc& d) {
   if (d.k == 0) {                                                  // dense all-pairs: tc_pair_kernel<lean | generic>
     if (f.QT > TP_QMAX) return EGNN_ERR_UNSUPPORTED;
     const size_t smem = pair_is_lean(f) ? tc_pair_smem_bytes<false>(f.Hp, 1) : tc_pair_smem_bytes<true>(f.Hp, f.QT, 1 + 2 * f.s.F);
-    if (smem > 227 * 1024) return EGNN_ERR_UNSUPPORTED;
+    if (smem > TC_SMEM_MAX) return EGNN_ERR_UNSUPPORTED;
   } else {                                                         // neighbour lists: tc_knn_kernel<lean | edges | generic>
     if (d.k > 32) return EGNN_ERR_UNSUPPORTED;
     const int mode = knn_mode(f);
     if (mode == TK_GEN && f.QT > TP_QMAX) return EGNN_ERR_UNSUPPORTED;
-    if (tc_knn_smem_bytes(f.Hp, mode, f.QT) > 227 * 1024) return EGNN_ERR_UNSUPPORTED;
+    if (tc_knn_smem_bytes(f.Hp, mode, f.QT) > TC_SMEM_MAX) return EGNN_ERR_UNSUPPORTED;
   }
   return EGNN_OK;
 }
@@ -207,51 +199,20 @@ struct FastWs { size_t Atab, Btab, node_in, h1, nbr_idx, nbr_ok, gpart, gcount, 
 constexpr int TP_JSPLIT_MAX = 8;
 FastWs fast_ws_layout(const FastDims& f, uint32_t flags) {
   FastWs w;
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t r = o; o += round_up(bytes, 256); return r; };
+  BumpAlloc o;
   const bool uf = flags & EGNN_FLAG_UPDATE_FEATS;
-  w.Atab = take((size_t)f.s.M * f.Hp * 4);
-  w.Btab = take(((size_t)f.s.M + 128) * f.Hp * 2);      // +128 rows: the dense kernel reads (and discards) up to a tile past the end
-  w.node_in = take(uf ? (size_t)f.s.M * f.Kn * 2 : 0);
-  w.h1 = take(uf ? (size_t)f.s.M * 2 * f.s.dim * 2 : 0);
-  w.nbr_idx = take((size_t)f.s.M * f.s.k * sizeof(int32_t));
-  w.nbr_ok = take((size_t)f.s.M * f.s.k);
+  w.Atab = o.take((size_t)f.s.M * f.Hp * 4);
+  w.Btab = o.take(((size_t)f.s.M + 128) * f.Hp * 2);    // +128 rows: the dense kernel reads (and discards) up to a tile past the end
+  w.node_in = o.take(uf ? (size_t)f.s.M * f.Kn * 2 : 0);
+  w.h1 = o.take(uf ? (size_t)f.s.M * 2 * f.s.dim * 2 : 0);
+  w.nbr_idx = o.take((size_t)f.s.M * f.s.k * sizeof(int32_t));
+  w.nbr_ok = o.take((size_t)f.s.M * f.s.k);
   // dense kernel, j-split mode: partial sums and arrival counters per row group (the counters are kept zero between calls)
   const size_t rgs = f.s.k == 0 ? (size_t)f.s.B * ceil_div(f.s.row1 - f.s.row0, TP_TI) : 0;
-  w.gpart = take(rgs * TP_JSPLIT_MAX * TP_TI * TpCfg<true>::PW * 8);
-  w.gcount = take(rgs * 4);
-  w.total = o;
+  w.gpart = o.take(rgs * TP_JSPLIT_MAX * TP_TI * TpCfg<true>::PW * 8);
+  w.gcount = o.take(rgs * 4);
+  w.total = o.total;
   return w;
-}
-
-// cudaFuncSetAttribute(MaxDynamicSharedMemorySize) once per (kernel, device), under a mutex: the only mutable
-// state of this file, written once per device and never shrunk.  TAG distinguishes kernels of identical type.
-template <int TAG, typename K>
-int ensure_dyn_smem(K kernel, size_t bytes) {
-  static std::mutex mu;
-  static size_t set[64] = {0};
-  int dev = 0;
-  EGNN_CUDA_TRY(cudaGetDevice(&dev));
-  std::lock_guard<std::mutex> lock(mu);
-  if (dev >= 64 || set[dev] < bytes) {
-    EGNN_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    if (dev < 64) set[dev] = bytes;
-  }
-  return EGNN_OK;
-}
-
-int sm_count(int* out) {
-  static std::mutex mu;
-  static int cached[64] = {0};
-  int dev = 0;
-  EGNN_CUDA_TRY(cudaGetDevice(&dev));
-  std::lock_guard<std::mutex> lock(mu);
-  if (dev < 64 && cached[dev] > 0) { *out = cached[dev]; return EGNN_OK; }
-  int n = 0;
-  EGNN_CUDA_TRY(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev));
-  if (dev < 64) cached[dev] = n;
-  *out = n;
-  return EGNN_OK;
 }
 
 // Optional start-up delay between the warpgroups of the persistent dense kernel (tc_pair.cuh), EGNN_B200_SKEW_NS.
@@ -269,17 +230,12 @@ uint32_t pair_skew_ns() {
 // one launch for one (g2 == nullptr) or two problems over the same rows
 int launch_tc_gemm(const TcGemmArgs& g, cudaStream_t st, const TcGemmArgs* g2 = nullptr) {
   if (g.M <= 0) return EGNN_OK;
-  EGNN_TRY((ensure_dyn_smem<0>(tc_gemm_kernel, GEMM_SMEM_BYTES)));
   TcGemmPair gp;
   gp.p[0] = g;
   gp.p[1] = g2 ? *g2 : g;
   gp.nt0 = ceil_div(g.Nout, GEMM_BN);
   const int nt1 = g2 ? ceil_div(g2->Nout, GEMM_BN) : 0;
-  dim3 grid(gp.nt0 + nt1, ceil_div(g.M, GEMM_BM));
-  tc_gemm_kernel<<<grid, 128, GEMM_SMEM_BYTES, st>>>(gp);
-  EGNN_LAUNCH_CHECK();
-  count_launch();
-  return EGNN_OK;
+  return launch_upto(TC_SMEM_MAX, tc_gemm_kernel, dim3(gp.nt0 + nt1, ceil_div(g.M, GEMM_BM)), 128, GEMM_SMEM_BYTES, st, gp);
 }
 
 }  // namespace
@@ -306,9 +262,7 @@ int fast_pack_weights(const EgnnLayerDesc& d, const EgnnLayerWeights& w, void* p
   const FastDims f = fast_dims(d);
   const FastPack L = fast_pack_layout(f);
   if (bytes < L.total) return EGNN_ERR_WORKSPACE;
-  fast_pack_kernel<<<296, 256, 0, st>>>(f, L, w, d.flags, static_cast<unsigned char*>(packed));
-  EGNN_LAUNCH_CHECK();
-  return EGNN_OK;
+  return launch(fast_pack_kernel, 296, 256, 0, st, f, L, w, d.flags, static_cast<unsigned char*>(packed));
 }
 
 int fast_workspace_bytes(const EgnnLayerDesc& d, size_t* out) {
@@ -350,13 +304,10 @@ int fast_forward(const EgnnLayerDesc& d, const EgnnLayerWeights& w, const void* 
       t.feats = feats; t.w1i = reinterpret_cast<const __nv_bfloat16*>(pk + L.w1i); t.w1j = reinterpret_cast<const __nv_bfloat16*>(pk + L.w1j);
       t.b1 = reinterpret_cast<const float*>(pk + L.b1); t.Atab = Atab; t.Btab = Btab;
       t.M = s.M; t.N = s.N; t.dim = s.dim; t.Hp = f.Hp; t.row0 = r0; t.row1 = r1;
-      const size_t smem = tables_small_smem(s.dim, f.Hp);
-      EGNN_TRY((ensure_dyn_smem<6>(tables_small_kernel, smem)));
       int sms = 0;
-      EGNN_TRY(sm_count(&sms));
-      tables_small_kernel<<<std::min(ceil_div(s.M, SN_WARPS), 4 * sms), SN_WARPS * 32, smem, st>>>(t);
-      EGNN_LAUNCH_CHECK();
-      count_launch();
+      EGNN_TRY(device_sm_count(&sms));
+      EGNN_TRY(launch_upto(TC_SMEM_MAX, tables_small_kernel, std::min(ceil_div(s.M, SN_WARPS), 4 * sms), SN_WARPS * 32,
+                           tables_small_smem(s.dim, f.Hp), st, t));
     } else {
       TcGemmArgs g{};
       g.lda = s.dim; g.K = s.dim; g.Nv = f.Hp; g.Nout = f.Hp; g.scale = 0.5f; g.act = 0; g.R = nullptr; g.ldr = 0; g.ldo = f.Hp;
@@ -400,7 +351,7 @@ int fast_forward(const EgnnLayerDesc& d, const EgnnLayerWeights& w, const void* 
     if (f.L > 0 && !io.edge_labels) return EGNN_ERR_NULL;
     if (s.edge_dim > 0 && !io.edges) return EGNN_ERR_NULL;
     int sms = 0;
-    EGNN_TRY(sm_count(&sms));
+    EGNN_TRY(device_sm_count(&sms));
     int items = s.B * ceil_div(R, TP_TI);
     if (items > 0) {
       // too few row groups to balance one CTA per SM: deal the j-blocks of every row group to 2 / 4 / 8 items
@@ -418,34 +369,15 @@ int fast_forward(const EgnnLayerDesc& d, const EgnnLayerWeights& w, const void* 
       }
       const int grid = items < sms ? items : sms;
       if (items < 2 * sms) a.skew_ns = 0;                      // too few row groups per CTA for the de-phasing to pay
-      if (pair_is_lean(f)) {
-        const size_t smem = tc_pair_smem_bytes<false>(f.Hp, 1);
-        EGNN_TRY((ensure_dyn_smem<1>(tc_pair_kernel<false>, smem)));
-        tc_pair_kernel<false><<<grid, TP_THREADS, smem, st>>>(a);
-      } else {
-        const size_t smem = tc_pair_smem_bytes<true>(f.Hp, f.QT, 1 + 2 * f.s.F);
-        EGNN_TRY((ensure_dyn_smem<2>(tc_pair_kernel<true>, smem)));
-        tc_pair_kernel<true><<<grid, TP_THREADS, smem, st>>>(a);
-      }
-      EGNN_LAUNCH_CHECK();
-      count_launch();
+      if (pair_is_lean(f))
+        EGNN_TRY(launch_upto(TC_SMEM_MAX, tc_pair_kernel<false>, grid, TP_THREADS, tc_pair_smem_bytes<false>(f.Hp, 1), st, a));
+      else
+        EGNN_TRY(launch_upto(TC_SMEM_MAX, tc_pair_kernel<true>, grid, TP_THREADS, tc_pair_smem_bytes<true>(f.Hp, f.QT, 1 + 2 * f.s.F), st, a));
     }
   } else {         // neighbour lists: distance + top-k select, then the gathered fused edge kernel
     int32_t* nbr_idx = reinterpret_cast<int32_t*>(base + wl.nbr_idx);
     uint8_t* nbr_ok = base + wl.nbr_ok;
-    if (io.nbr_idx) {                                  // edge-list mode: the caller's lists, no ranking
-      nbr_idx = const_cast<int32_t*>(io.nbr_idx);
-      nbr_ok = nullptr;
-    } else {
-      StageTimer tm(st, STAGE_SELECT);
-      const double vr = (d.flags & EGNN_FLAG_ONLY_SPARSE) ? 0.0 : d.valid_radius;
-      if ((d.flags & EGNN_FLAG_ONLY_SPARSE) && io.mask && io.adj)      // every slot top-k could add is masked out: row scan
-        EGNN_TRY(adj_neighbors_dispatch(s.B, s.N, s.k, io.adj, (d.flags & EGNN_FLAG_ADJ_BATCHED) ? 1 : 0, nbr_idx, nbr_ok, st));
-      else
-        EGNN_TRY(knn_select_dispatch(EGNN_DTYPE_F32, s.B, s.N, s.C, s.k, io.coors, io.mask, io.adj,
-                                     (d.flags & EGNN_FLAG_ADJ_BATCHED) ? 1 : 0, vr, nbr_idx, nbr_ok, st));
-      count_launch();
-    }
+    EGNN_TRY(select_neighbours(d, s, io, EGNN_DTYPE_F32, nbr_idx, nbr_ok, st));
     StageTimer tm(st, STAGE_PAIR);
     TcKnnArgs a{};
     a.B = s.B; a.N = s.N; a.Hp = f.Hp; a.ldn = f.Kn; a.dim = s.dim; a.k = s.k; a.edge_dim = s.edge_dim;
@@ -468,24 +400,11 @@ int fast_forward(const EgnnLayerDesc& d, const EgnnLayerWeights& w, const void* 
     const int mode = knn_mode(f);
     const int rows = tc_knn_rows_per_cta(f.Hp, mode, f.QT);         // 8 (two CTAs per SM) when shared memory allows
     const size_t smem = tc_knn_smem_bytes(f.Hp, mode, f.QT, rows);
-    dim3 grid(ceil_div(R, rows), s.B);
-    if (R > 0) {
-#define EGNN_TC_KNN_LAUNCH(TAG, MODE_, ROWS_)                                                  \
-  do {                                                                                          \
-    EGNN_TRY((ensure_dyn_smem<TAG>(tc_knn_kernel<MODE_, ROWS_>, smem)));                        \
-    tc_knn_kernel<MODE_, ROWS_><<<grid, ROWS_ * 32, smem, st>>>(a);                             \
-  } while (0)
-      if (mode == TK_LEAN) {
-        if (rows == 8) EGNN_TC_KNN_LAUNCH(3, TK_LEAN, 8); else EGNN_TC_KNN_LAUNCH(13, TK_LEAN, 16);
-      } else if (mode == TK_EDGES) {
-        if (rows == 8) EGNN_TC_KNN_LAUNCH(4, TK_EDGES, 8); else EGNN_TC_KNN_LAUNCH(14, TK_EDGES, 16);
-      } else {
-        if (rows == 8) EGNN_TC_KNN_LAUNCH(5, TK_GEN, 8); else EGNN_TC_KNN_LAUNCH(15, TK_GEN, 16);
-      }
-#undef EGNN_TC_KNN_LAUNCH
-      EGNN_LAUNCH_CHECK();
-      count_launch();
-    }
+    const bool r8 = rows == 8;
+    auto kernel = mode == TK_LEAN ? (r8 ? tc_knn_kernel<TK_LEAN, 8> : tc_knn_kernel<TK_LEAN, 16>)
+                : mode == TK_EDGES ? (r8 ? tc_knn_kernel<TK_EDGES, 8> : tc_knn_kernel<TK_EDGES, 16>)
+                                   : (r8 ? tc_knn_kernel<TK_GEN, 8> : tc_knn_kernel<TK_GEN, 16>);
+    if (R > 0) EGNN_TRY(launch_upto(TC_SMEM_MAX, kernel, dim3(ceil_div(R, rows), s.B), rows * 32, smem, st, a));
   }
   StageTimer post(st, STAGE_NODE_POST);
   __nv_bfloat16* fout = static_cast<__nv_bfloat16*>(io.feats_out);
@@ -497,21 +416,16 @@ int fast_forward(const EgnnLayerDesc& d, const EgnnLayerWeights& w, const void* 
       n.bn2 = reinterpret_cast<const float*>(pk + L.bn2); n.lng = reinterpret_cast<const float*>(pk + L.lng);
       n.lnb = reinterpret_cast<const float*>(pk + L.lnb); n.out = fout;
       n.B = s.B; n.N = s.N; n.dim = s.dim; n.Kn = f.Kn; n.m = s.m; n.row0 = r0; n.row1 = r1; n.do_norm = (d.flags & EGNN_FLAG_NORM_FEATS) ? 1 : 0;
-      const size_t smem = node_small_smem(s.dim, f.Kn);
-      EGNN_TRY((ensure_dyn_smem<7>(node_update_small_kernel, smem)));
       int sms = 0;
-      EGNN_TRY(sm_count(&sms));
-      node_update_small_kernel<<<std::min(ceil_div(s.B * R, SN_WARPS), 4 * sms), SN_WARPS * 32, smem, st>>>(n);
-      EGNN_LAUNCH_CHECK();
-      count_launch();
+      EGNN_TRY(device_sm_count(&sms));
+      EGNN_TRY(launch_upto(TC_SMEM_MAX, node_update_small_kernel, std::min(ceil_div(s.B * R, SN_WARPS), 4 * sms), SN_WARPS * 32,
+                           node_small_smem(s.dim, f.Kn), st, n));
     } else
     for (int sg = 0; sg < nseg; ++sg) {
       const size_t o = seg_begin(sg);
-      ln_concat_bf16_kernel<<<ceil_div(seg_rows * 32, 256), 256, 0, st>>>(
-          feats + o * s.dim, reinterpret_cast<const float*>(pk + L.lng), reinterpret_cast<const float*>(pk + L.lnb),
-          node_in + o * f.Kn, f.Kn, s.dim, s.m, seg_rows, (d.flags & EGNN_FLAG_NORM_FEATS) ? 1 : 0);
-      EGNN_LAUNCH_CHECK();
-      count_launch();
+      EGNN_TRY(launch(ln_concat_bf16_kernel, ceil_div(seg_rows * 32, 256), 256, 0, st, feats + o * s.dim,
+                      reinterpret_cast<const float*>(pk + L.lng), reinterpret_cast<const float*>(pk + L.lnb), node_in + o * f.Kn,
+                      f.Kn, s.dim, s.m, seg_rows, (d.flags & EGNN_FLAG_NORM_FEATS) ? 1 : 0));
       TcGemmArgs g{};
       g.A = node_in + o * f.Kn; g.lda = f.Kn; g.K = f.Kn; g.M = seg_rows; g.Nv = 2 * s.dim; g.Nout = 2 * s.dim; g.scale = 1.f; g.act = 1;
       g.W = reinterpret_cast<const __nv_bfloat16*>(pk + L.wn1); g.ldw = f.Kn;

@@ -143,14 +143,14 @@ __global__ void ga_add_kernel(const T* __restrict__ a, const T* __restrict__ b, 
 struct GaWs { size_t xn, qn, q1, kv1, S, o1, induced, q2, kv2, o2, x1, hff, total; };
 GaWs ga_layout(const EgnnGlobalAttnDesc& d, size_t es) {
   GaWs w;
-  size_t o = 0;
-  auto take = [&](size_t elems) { size_t r = o; o += round_up(elems * es, 256); return r; };
+  BumpAlloc o;
+  auto take = [&](size_t elems) { return o.take(elems * es); };
   const size_t BN = (size_t)d.B * d.N, BT = (size_t)d.B * d.T, inner = (size_t)d.heads * d.dim_head;
   w.xn = take(BN * d.dim); w.qn = take(BT * d.dim); w.q1 = take(BT * inner); w.kv1 = take(BN * 2 * inner);
   w.S = take((size_t)d.B * d.heads * d.T * d.N); w.o1 = take(BT * inner); w.induced = take(BT * d.dim);
   w.q2 = take(BN * inner); w.kv2 = take(BT * 2 * inner); w.o2 = take(BN * inner); w.x1 = take(BN * d.dim);
   w.hff = take(BN * 4 * d.dim);
-  w.total = o;
+  w.total = o.total;
   return w;
 }
 
@@ -176,33 +176,27 @@ int ga_forward(const EgnnGlobalAttnDesc& d, const EgnnGlobalAttnWeights& w, cons
   const T* qs = W(io.queries);
   const RowMap idn{BN, BN, 0}, idt{BT, BT, 0};
   // x, queries = norm_seq(x), norm_queries(queries)                              :134
-  ga_layernorm_kernel<T><<<ceil_div(BN * 32, 256), 256, 0, st>>>(x, W(w.norm_seq_g), W(w.norm_seq_b), P(L.xn), BN, dim);
-  ga_layernorm_kernel<T><<<ceil_div(BT * 32, 256), 256, 0, st>>>(qs, W(w.norm_q_g), W(w.norm_q_b), P(L.qn), BT, dim);
-  EGNN_LAUNCH_CHECK();
+  EGNN_TRY(launch(ga_layernorm_kernel<T>, ceil_div(BN * 32, 256), 256, 0, st, x, W(w.norm_seq_g), W(w.norm_seq_b), P(L.xn), BN, dim));
+  EGNN_TRY(launch(ga_layernorm_kernel<T>, ceil_div(BT * 32, 256), 256, 0, st, qs, W(w.norm_q_g), W(w.norm_q_b), P(L.qn), BT, dim));
   // induced = attn1(queries, x, mask)                                            :136
   EGNN_TRY((launch_gemm<T, 0, false>(P(L.qn), dim, W(w.a1_wq), dim, nullptr, nullptr, 0, P(L.q1), inner, BT, inner, inner, dim, idt, st)));
   EGNN_TRY((launch_gemm<T, 0, false>(P(L.xn), dim, W(w.a1_wkv), dim, nullptr, nullptr, 0, P(L.kv1), 2 * inner, BN, 2 * inner, 2 * inner, dim, idn, st)));
-  {
-    const size_t total = (size_t)d.B * d.heads * d.T * d.N;
-    ga_scores_kernel<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(P(L.q1), P(L.kv1), io.mask, P(L.S), d.B, d.N, d.T, d.heads, d.dim_head, scale);
-    ga_softmax_av_kernel<T><<<dim3(d.T, d.heads, d.B), 256, 0, st>>>(P(L.S), P(L.kv1), P(L.o1), d.N, d.T, d.heads, d.dim_head);
-    EGNN_LAUNCH_CHECK();
-  }
+  const size_t scores = (size_t)d.B * d.heads * d.T * d.N;
+  EGNN_TRY(launch(ga_scores_kernel<T>, (unsigned)((scores + 255) / 256), 256, 0, st, P(L.q1), P(L.kv1), io.mask, P(L.S), d.B, d.N, d.T,
+                  d.heads, d.dim_head, scale));
+  EGNN_TRY(launch(ga_softmax_av_kernel<T>, dim3(d.T, d.heads, d.B), 256, 0, st, P(L.S), P(L.kv1), P(L.o1), d.N, d.T, d.heads, d.dim_head));
   EGNN_TRY((launch_gemm<T, 0, false>(P(L.o1), inner, W(w.a1_wo), inner, W(w.a1_bo), nullptr, 0, P(L.induced), dim, BT, dim, dim, inner, idt, st)));
   // out = attn2(x, induced);  x = out + res_x                                     :137, :139
   EGNN_TRY((launch_gemm<T, 0, false>(P(L.xn), dim, W(w.a2_wq), dim, nullptr, nullptr, 0, P(L.q2), inner, BN, inner, inner, dim, idn, st)));
   EGNN_TRY((launch_gemm<T, 0, false>(P(L.induced), dim, W(w.a2_wkv), dim, nullptr, nullptr, 0, P(L.kv2), 2 * inner, BT, 2 * inner, 2 * inner, dim, idt, st)));
-  {
-    const size_t warps = (size_t)BN * d.heads;
-    ga_attn2_kernel<T><<<(unsigned)((warps * 32 + 255) / 256), 256, 0, st>>>(P(L.q2), P(L.kv2), P(L.o2), d.B, d.N, d.T, d.heads, d.dim_head, scale);
-    EGNN_LAUNCH_CHECK();
-  }
+  const size_t warps = (size_t)BN * d.heads;
+  EGNN_TRY(launch(ga_attn2_kernel<T>, (unsigned)((warps * 32 + 255) / 256), 256, 0, st, P(L.q2), P(L.kv2), P(L.o2), d.B, d.N, d.T, d.heads,
+                  d.dim_head, scale));
   EGNN_TRY((launch_gemm<T, 0, true>(P(L.o2), inner, W(w.a2_wo), inner, W(w.a2_bo), x, dim, P(L.x1), dim, BN, dim, dim, inner, idn, st)));
   // queries = induced + res_queries                                              :140
-  ga_add_kernel<T><<<ceil_div(BT * dim, 256), 256, 0, st>>>(P(L.induced), qs, static_cast<T*>(io.queries_out), (size_t)BT * dim);
+  EGNN_TRY(launch(ga_add_kernel<T>, ceil_div(BT * dim, 256), 256, 0, st, P(L.induced), qs, static_cast<T*>(io.queries_out), (size_t)BT * dim));
   // x = ff(x) + x                                                                :142
-  ga_layernorm_kernel<T><<<ceil_div(BN * 32, 256), 256, 0, st>>>(P(L.x1), W(w.ff_ln_g), W(w.ff_ln_b), P(L.xn), BN, dim);
-  EGNN_LAUNCH_CHECK();
+  EGNN_TRY(launch(ga_layernorm_kernel<T>, ceil_div(BN * 32, 256), 256, 0, st, P(L.x1), W(w.ff_ln_g), W(w.ff_ln_b), P(L.xn), BN, dim));
   EGNN_TRY((launch_gemm<T, 2, false>(P(L.xn), dim, W(w.ff_w1), dim, W(w.ff_b1), nullptr, 0, P(L.hff), 4 * dim, BN, 4 * dim, 4 * dim, dim, idn, st)));
   EGNN_TRY((launch_gemm<T, 0, true>(P(L.hff), 4 * dim, W(w.ff_w2), 4 * dim, W(w.ff_b2), P(L.x1), dim, static_cast<T*>(io.x_out), dim, BN, dim, dim,
                                     4 * dim, idn, st)));

@@ -12,7 +12,8 @@
 // beat the current k-th entry are queued in shared memory and merged 32 at a time with a
 // warp-bitonic sort + merge, so the O(N^2) ranking matrix is never written.
 // k  > 32: one block per row sorts all N (rank, j) pairs in shared memory (bitonic).
-#include "common.cuh"
+#include "knn_select.h"
+#include "launch.cuh"
 
 namespace egnn {
 
@@ -244,44 +245,24 @@ static int launch_select(int B, int N, int C, int k, const void* coors, const ui
   a.mask = mask; a.adj = adj; a.adj_batched = adj_batched;
   a.valid_radius = (T)valid_radius;
   a.out_idx = out_idx; a.out_ok = out_ok;
-  const int rows = B * N;
   if (k <= 32) {
-    static bool attr_set[64] = {false};
-    int dev = 0;
-    EGNN_CUDA_TRY(cudaGetDevice(&dev));
-    if (dev < 64 && !attr_set[dev]) {
-      EGNN_CUDA_TRY(cudaFuncSetAttribute(knn_warp_select_kernel<T, 16, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)sel_smem_bytes<T>(8, 16)));
-      EGNN_CUDA_TRY(cudaFuncSetAttribute(knn_warp_select_kernel<T, 8, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)sel_smem_bytes<T>(8, 8)));
-      attr_set[dev] = true;
-    }
     // 16 rows per CTA halve the staging work per row; small problems keep 8 so that more SMs take part
     const bool wide = (long)B * ceil_div(N, 16) >= 296;
-    dim3 grid(ceil_div(N, wide ? 16 : 8), B);
-    const size_t smem = sel_smem_bytes<T>(C, wide ? 16 : 8);
-    if (C == 3) {
-      if (wide) knn_warp_select_kernel<T, 16, 3><<<grid, 16 * 32, smem, st>>>(a);
-      else knn_warp_select_kernel<T, 8, 3><<<grid, 8 * 32, smem, st>>>(a);
-    } else {
-      if (wide) knn_warp_select_kernel<T, 16, 0><<<grid, 16 * 32, smem, st>>>(a);
-      else knn_warp_select_kernel<T, 8, 0><<<grid, 8 * 32, smem, st>>>(a);
-    }
-  } else {
-    int Npad = 1;
-    while (Npad < N) Npad <<= 1;
-    const size_t smem = (size_t)Npad * (sizeof(T) + sizeof(int));
-    if (smem > 200 * 1024) return EGNN_ERR_UNSUPPORTED;     // N too large for the k>32 path
-    EGNN_CUDA_TRY(cudaFuncSetAttribute(knn_block_sort_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    knn_block_sort_kernel<T><<<rows, 256, smem, st>>>(a, Npad);
+    const int warps = wide ? 16 : 8;
+    auto kernel = C == 3 ? (wide ? knn_warp_select_kernel<T, 16, 3> : knn_warp_select_kernel<T, 8, 3>)
+                         : (wide ? knn_warp_select_kernel<T, 16, 0> : knn_warp_select_kernel<T, 8, 0>);
+    return launch(kernel, dim3(ceil_div(N, warps), B), warps * 32, sel_smem_bytes<T>(C, warps), st, a);
   }
-  EGNN_LAUNCH_CHECK();
-  return EGNN_OK;
+  int Npad = 1;
+  while (Npad < N) Npad <<= 1;
+  const size_t smem = (size_t)Npad * (sizeof(T) + sizeof(int));
+  if (smem > 200 * 1024) return EGNN_ERR_UNSUPPORTED;     // N too large for the k>32 path
+  return launch(knn_block_sort_kernel<T>, B * N, 256, smem, st, a, Npad);
 }
 
-int knn_select_dispatch(int32_t dtype, int B, int N, int C, int k, const void* coors, const uint8_t* mask,
-                        const uint8_t* adj, int adj_batched, double valid_radius, int32_t* out_idx,
-                        uint8_t* out_ok, cudaStream_t st) {
+static int knn_select_dispatch(int32_t dtype, int B, int N, int C, int k, const void* coors, const uint8_t* mask,
+                               const uint8_t* adj, int adj_batched, double valid_radius, int32_t* out_idx,
+                               uint8_t* out_ok, cudaStream_t st) {
   if (!coors || !out_idx) return EGNN_ERR_NULL;
   if (B <= 0 || B > 65535 || N <= 0 || C <= 0 || C > 8 || k <= 0 || k > N) return EGNN_ERR_SHAPE;
   if (dtype == EGNN_DTYPE_F64)
@@ -341,14 +322,27 @@ __global__ void __launch_bounds__(256) adj_neighbors_kernel(int B, int N, int k,
   for (int p = pos + lane; p < k; p += 32) { oi[p] = ok ? i : -1; if (ok) ok[p] = 0; }
 }
 
-int adj_neighbors_dispatch(int B, int N, int k, const uint8_t* adj, int adj_batched, int32_t* out_idx, uint8_t* out_ok,
-                           cudaStream_t st) {
+static int adj_neighbors_dispatch(int B, int N, int k, const uint8_t* adj, int adj_batched, int32_t* out_idx,
+                                  uint8_t* out_ok, cudaStream_t st) {
   if (!adj || !out_idx) return EGNN_ERR_NULL;
   if (B <= 0 || N <= 0 || k <= 0 || k > N) return EGNN_ERR_SHAPE;
   const long long threads = (long long)B * N * 32;
-  adj_neighbors_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(B, N, k, adj, adj_batched, out_idx, out_ok);
-  EGNN_LAUNCH_CHECK();
-  return EGNN_OK;
+  return launch(adj_neighbors_kernel, (unsigned)((threads + 255) / 256), 256, 0, st, B, N, k, adj, adj_batched, out_idx, out_ok);
+}
+
+int select_neighbours(const EgnnLayerDesc& d, const Dims& s, const EgnnLayerIO& io, int32_t coors_dtype, int32_t*& idx,
+                      uint8_t*& ok, cudaStream_t st) {
+  if (io.nbr_idx) {                                  // edge-list mode: the caller's lists, no ranking
+    idx = const_cast<int32_t*>(io.nbr_idx);
+    ok = nullptr;
+    return EGNN_OK;
+  }
+  StageTimer tm(st, STAGE_SELECT);
+  const int adj_batched = (d.flags & EGNN_FLAG_ADJ_BATCHED) ? 1 : 0;
+  if ((d.flags & EGNN_FLAG_ONLY_SPARSE) && io.mask && io.adj)      // every slot top-k could add is masked out: row scan
+    return adj_neighbors_dispatch(s.B, s.N, s.k, io.adj, adj_batched, idx, ok, st);
+  const double vr = (d.flags & EGNN_FLAG_ONLY_SPARSE) ? 0.0 : d.valid_radius;     // :250
+  return knn_select_dispatch(coors_dtype, s.B, s.N, s.C, s.k, io.coors, io.mask, io.adj, adj_batched, vr, idx, ok, st);
 }
 
 }  // namespace egnn

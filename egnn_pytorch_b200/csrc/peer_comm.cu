@@ -9,7 +9,7 @@
 // Buffers are double-buffered by epoch parity: a rank that is one call ahead writes the OTHER half, and it cannot be
 // two calls ahead because call n+1 waits for every peer's epoch-(n+1) flag, which a peer only raises after it
 // finished (stream order) everything that read the epoch-(n-1) half.
-#include "common.cuh"
+#include "launch.cuh"
 #include <string.h>
 #include <new>
 
@@ -173,9 +173,7 @@ int egnn_comm_allgather(void* comm, int32_t nseg, const void* const* src, const 
   }
   int ctas = (int)((most / 16 + 255) / 256);
   ctas = ctas < 1 ? 1 : (ctas > 16 ? 16 : ctas);                 // NVLink is saturated by a handful of CTAs per peer
-  dim3 grid(ctas, c->world);
-  egnn::peer_push_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(a);
-  EGNN_LAUNCH_CHECK();
+  EGNN_TRY(egnn::launch(egnn::peer_push_kernel, dim3(ctas, c->world), 256, 0, static_cast<cudaStream_t>(stream), a));
   *gathered_out = c->local + a.half_off;
   return EGNN_OK;
 }

@@ -35,9 +35,9 @@ struct StageTimer {
   }
 };
 
-inline void count_launch(int n = 1) {
+inline void count_launch() {
   Profiler& p = Profiler::get();
-  if (p.on) { std::lock_guard<std::mutex> g(p.mu); p.launches += n; }
+  if (p.on) { std::lock_guard<std::mutex> g(p.mu); p.launches += 1; }
 }
 
 }  // namespace egnn

@@ -3,7 +3,7 @@
 #pragma once
 #include "common.cuh"
 #include "simt_kernels.cuh"
-#include "profile.h"
+#include "launch.cuh"
 #include <algorithm>
 
 namespace egnn {
@@ -46,35 +46,17 @@ static int simt_hsplit(const Dims& s) {
 }
 static SimtWs simt_ws_layout(const Dims& s, size_t es, uint32_t flags) {
   SimtWs w;
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t r = o; o += round_up(bytes, 256); return r; };
-  w.P = take((size_t)s.M * 2 * s.Hp * es);
+  BumpAlloc o;
+  w.P = o.take((size_t)s.M * 2 * s.Hp * es);
   const bool uf = flags & EGNN_FLAG_UPDATE_FEATS;
-  w.node_in = take(uf ? (size_t)s.M * (s.dim + s.m) * es : 0);
-  w.h1 = take(uf ? (size_t)s.M * 2 * s.dim * es : 0);
-  w.nbr_idx = take((size_t)s.M * s.k * sizeof(int32_t));
-  w.nbr_ok = take((size_t)s.M * s.k);
+  w.node_in = o.take(uf ? (size_t)s.M * (s.dim + s.m) * es : 0);
+  w.h1 = o.take(uf ? (size_t)s.M * 2 * s.dim * es : 0);
+  w.nbr_idx = o.take((size_t)s.M * s.k * sizeof(int32_t));
+  w.nbr_ok = o.take((size_t)s.M * s.k);
   w.hsplit = simt_hsplit(s);
-  w.hpart = take(w.hsplit > 1 ? (size_t)w.hsplit * s.B * s.N * s.N * 32 * es : 0);
-  w.total = o;
+  w.hpart = o.take(w.hsplit > 1 ? (size_t)w.hsplit * s.B * s.N * s.N * 32 * es : 0);
+  w.total = o.total;
   return w;
-}
-
-// Largest dynamic shared memory any SIMT kernel opts in to.  The backward preflight (backward_supported) checks its
-// kernels' sizes against the same constant, so a configuration it accepts cannot fail here at launch time.
-constexpr size_t DYN_SMEM_MAX = 220 * 1024;
-
-// Opt a kernel in to `smem` bytes of dynamic shared memory.  The attribute is read back first and only ever raised:
-// the same kernel template is launched from several translation units, so no TU-local cache may lower it.
-template <typename K>
-static int ensure_dynamic_smem(K kernel, size_t smem) {
-  if (smem > DYN_SMEM_MAX) return EGNN_ERR_UNSUPPORTED;
-  if (smem <= 48 * 1024) return EGNN_OK;
-  cudaFuncAttributes attr;
-  EGNN_CUDA_TRY(cudaFuncGetAttributes(&attr, kernel));
-  if ((size_t)attr.maxDynamicSharedSizeBytes < smem)
-    EGNN_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  return EGNN_OK;
 }
 
 template <typename T, int ACT, bool RES>
@@ -85,26 +67,12 @@ static int launch_gemm(const T* A, int lda, const T* W, int ldw, const T* bias, 
   if (Mr <= 16 && skinny_smem <= 96 * 1024) {
     // columns per warp: as many as still give about one CTA per SM (the kernel is bound by weight streaming)
     const int cols = Nout >= 148 * SKINNY_WARPS * 4 ? 4 : (Nout >= 148 * SKINNY_WARPS * 2 ? 2 : 1);
-    const int grid = ceil_div(Nout, SKINNY_WARPS * cols);
-    if (cols == 4) {
-      EGNN_TRY(ensure_dynamic_smem(gemm_skinny_kernel<T, ACT, RES, 4>, skinny_smem));
-      gemm_skinny_kernel<T, ACT, RES, 4><<<grid, SKINNY_WARPS * 32, skinny_smem, st>>>(A, lda, W, ldw, bias, R, ldr, C, ldo, Mr, Nv, Nout, K, map, drop);
-    } else if (cols == 2) {
-      EGNN_TRY(ensure_dynamic_smem(gemm_skinny_kernel<T, ACT, RES, 2>, skinny_smem));
-      gemm_skinny_kernel<T, ACT, RES, 2><<<grid, SKINNY_WARPS * 32, skinny_smem, st>>>(A, lda, W, ldw, bias, R, ldr, C, ldo, Mr, Nv, Nout, K, map, drop);
-    } else {
-      EGNN_TRY(ensure_dynamic_smem(gemm_skinny_kernel<T, ACT, RES, 1>, skinny_smem));
-      gemm_skinny_kernel<T, ACT, RES, 1><<<grid, SKINNY_WARPS * 32, skinny_smem, st>>>(A, lda, W, ldw, bias, R, ldr, C, ldo, Mr, Nv, Nout, K, map, drop);
-    }
-    EGNN_LAUNCH_CHECK();
-    count_launch();
-    return EGNN_OK;
+    auto kernel = cols == 4 ? gemm_skinny_kernel<T, ACT, RES, 4> : cols == 2 ? gemm_skinny_kernel<T, ACT, RES, 2> : gemm_skinny_kernel<T, ACT, RES, 1>;
+    return launch(kernel, ceil_div(Nout, SKINNY_WARPS * cols), SKINNY_WARPS * 32, skinny_smem, st, A, lda, W, ldw, bias, R, ldr, C, ldo, Mr,
+                  Nv, Nout, K, map, drop);
   }
-  dim3 grid(ceil_div(Nout, 64), ceil_div(Mr, 64));
-  gemm_nt_kernel<T, ACT, RES><<<grid, 256, 0, st>>>(A, lda, W, ldw, bias, R, ldr, C, ldo, Mr, Nv, Nout, K, map, drop);
-  EGNN_LAUNCH_CHECK();
-  count_launch();
-  return EGNN_OK;
+  return launch(gemm_nt_kernel<T, ACT, RES>, dim3(ceil_div(Nout, 64), ceil_div(Mr, 64)), 256, 0, st, A, lda, W, ldw, bias, R, ldr, C, ldo,
+                Mr, Nv, Nout, K, map, drop);
 }
 
 static int check_ptrs(const EgnnLayerDesc& d, const EgnnLayerWeights* w, const EgnnLayerIO* io) {

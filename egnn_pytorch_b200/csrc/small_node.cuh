@@ -24,15 +24,6 @@ constexpr size_t SMALL_NODE_SMEM_MAX = 160 * 1024;   // staged weights beyond th
 constexpr int SN_TABLES_M_MAX = 4096;                // the table kernel re-reads its weights per node (28 % FMA density): measured
                                                      // faster than the GEMMs at 1024 nodes (12 vs 20 us), slower at 8192 (35 vs 21 us)
 
-inline int small_node_sms() {
-  static int sms = 0;
-  if (!sms) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) sms = 148;
-  }
-  return sms;
-}
-
 struct TablesSmallArgs {
   const __nv_bfloat16* feats;      // [M][dim]
   const __nv_bfloat16* w1i;        // [Hp][dim]

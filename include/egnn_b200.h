@@ -15,8 +15,8 @@
  *    outlives the call and never synchronises the stream (HOST-buffer entry excepted);
  *  - every entry returns 0 on success or a negative EGNN_ERR_* code and never throws;
  *  - all tensors are contiguous, row-major, in the layouts written next to each field;
- *  - re-entrant across streams and devices; the only mutable global state is a mutex-guarded, write-once per-device
- *    cache of kernel attributes / SM counts and the opt-in profiler below.
+ *  - re-entrant across streams and devices; the only mutable global state is one mutex-guarded per-device cache of
+ *    kernel shared-memory opt-ins (only ever raised) and SM counts, and the opt-in profiler below.
  */
 #ifndef EGNN_B200_H_
 #define EGNN_B200_H_
@@ -296,9 +296,10 @@ int egnn_comm_destroy(void* comm);
 
 /* Diagnostics for benchmarks: when enabled, every egnn_layer_forward brackets its stages
  * (0 neighbour select, 1 per-node tables, 2 fused edge kernel, 3 node update) with CUDA events
- * on the launch stream and counts kernel launches.  egnn_profile_read synchronises those events
- * and returns the accumulated milliseconds / span counts per stage (arrays of 4) and the launch
- * count.  Off by default; the only mutable global state in the library. */
+ * on the launch stream, and the library counts every kernel it launches, from any entry point
+ * (forward, backward, weight packing, adjacency, embedding, global attention, all-gather).
+ * egnn_profile_read synchronises those events and returns the accumulated milliseconds / span
+ * counts per stage (arrays of 4) and the launch count.  Off by default. */
 int egnn_profile_enable(int on);
 int egnn_profile_read(float* ms_out, int32_t* spans_out, int64_t* launches_out, int reset);
 
